@@ -14,6 +14,8 @@ N > 1 (weak scaling): every rank holds the SRS and runs its own 2^16-point slice
 partials stay on the device as c slice sums (128 B each), are exchanged with one NCCL all_gather enqueued behind the kernels and
 summed on the device (proof_systems_b200/parallel.py: ShardedMsm).  NTT: N independent replicas.
 Between timed iterations a 256 MiB buffer is overwritten to flush the 126 MB L2.
+--dump-outputs DIR writes what the last timed step returned (see dump_outputs), so that two builds can be compared on identical
+inputs: every input is derived from fixed seeds and the fixture's SRS.
 """
 import argparse
 import json
@@ -26,6 +28,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the tree may be read-only: nothing is written there
 
 LOG_N = 16
 N_PTS = 1 << LOG_N
@@ -131,8 +134,10 @@ def splitmix64_limbs(seed, n):
 
 
 def compressed_srs():
-    """the reference's own srs/pallas.srs generators (compressed, 33 B each), via tests/golden"""
-    return np.load(os.path.join(ROOT, "tests", "golden", "pallas_srs.npz"))["g_cmp"]
+    """the reference's own srs/pallas.srs generators (compressed, 33 B each), rebuilt by tests/golden/srs_fixture.py"""
+    sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
+    import srs_fixture
+    return srs_fixture.load("pallas")["g_cmp"]
 
 
 def make_inputs(decompress, rank):
@@ -142,6 +147,22 @@ def make_inputs(decompress, rank):
     scalars = splitmix64_limbs(1 + rank, N_PTS)      # canonical (msm_bigint form)
     poly = splitmix64_limbs(2, N_PTS)                # Montgomery residues
     return g, scalars, poly
+
+
+def field_digits(limbs: np.ndarray) -> np.ndarray:
+    """u64 limbs [..., 4] of 256-bit values -> float32 [..., 16]: 16 little-endian 16-bit digits per value, exact in float32"""
+    return np.ascontiguousarray(limbs, dtype=np.uint64).view(np.uint16).astype(np.float32)
+
+
+def dump_outputs(out_dir, msm_affine, ntt_out):
+    """The headline's last timed step, as float32 digits (field_digits) of the library's Montgomery limbs:
+      msm.npy  [2, 16]       the 2^16-point Pallas MSM, converted from the returned Jacobian point to affine (x, y) so that
+                             equal points compare equal
+      ntt.npy  [2^16, 16]    the polynomial the in-place Fp NTT left on the device (the step transforms the previous step's
+                             output: after W warm-up and K timed steps it holds NTT^(W+K) of the seeded input)"""
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "msm.npy"), field_digits(np.asarray(msm_affine).reshape(2, 4)))
+    np.save(os.path.join(out_dir, "ntt.npy"), field_digits(ntt_out))
 
 
 def cpu_time(fn, min_seconds, max_reps):
@@ -234,7 +255,12 @@ def main():
     ap.add_argument("--window-bits", type=int, default=16, help="table window of the resident SRS for the headline (16 = BASELINE config 2's w; -1: library default)")
     ap.add_argument("--cpu-seconds", type=float, default=6.0, help="budget of the cpu_baseline leg")
     ap.add_argument("--no-extra", action="store_true", help="skip the cfg1 / cfg3 / cfg4 legs (tools/ use this for quick A/B runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy (CUDA arm)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the CUDA arm")
     if args.warmup < 3:
         args.warmup = 3
     if args.impl == "reference":
@@ -354,9 +380,18 @@ def main():
         ntt_e2e()
     barrier()
     launches0 = ctx.launch_count
-    msm_ms = timed(step_resident, args.steps, collective=True)
+    last = {}
+
+    def step_resident_kept():
+        last["msm"] = step_resident()
+
+    msm_ms = timed(step_resident_kept, args.steps, collective=True)
+    result = last["msm"]
     barrier()
     ntt_ms = timed(ntt_resident, args.steps)
+    if args.dump_outputs:
+        stream.synchronize()
+        last["ntt"] = d_poly.cpu().numpy().view(np.uint64).reshape(N_PTS, 4).copy()
     barrier()
     msm_e2e_ms = timed(step_e2e, args.steps, collective=True)
     barrier()
@@ -468,7 +503,7 @@ def main():
         d_sc4 = torch.from_numpy(sc4[lo:hi].view(np.int64)).cuda()
         h_sc4 = torch.from_numpy(sc4[lo:hi].view(np.int64).copy()).pin_memory()
         sh4 = comm.msm if comm else (lambda bb, ptr, cnt: ctx.msm_dev(bb, ptr, cnt) if ptr == d_sc4.data_ptr() else msm_host(bb, h_sc4, cnt))
-        steps4 = max(3, min(args.steps, 10))
+        steps4 = args.steps
         for _ in range(3):
             r4 = sh4(b4, d_sc4.data_ptr(), hi - lo)
         barrier()
@@ -573,6 +608,8 @@ def main():
         },
         "extra": extra,
     }
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, zk.jacobian_to_affine(zk.PALLAS, result), last["ntt"])
     print(json.dumps(line))
     if world > 1:
         dist.destroy_process_group()

@@ -10,6 +10,9 @@ if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
 GOLDEN = os.path.join(ROOT, "tests", "golden")
+if GOLDEN not in sys.path:
+    sys.path.insert(0, GOLDEN)
+import srs_fixture  # noqa: E402
 
 
 def pytest_configure(config):
@@ -30,7 +33,7 @@ class GoldenSRS:
         self.cid = orc.PALLAS if curve_name == "pallas" else orc.VESTA
         self.base = orc.BASE_FIELD[self.cid]
         self.scalar = orc.SCALAR_FIELD[self.cid]
-        z = np.load(os.path.join(GOLDEN, f"{curve_name}_srs.npz"))
+        z = srs_fixture.load(curve_name)
         self.g_cmp = z["g_cmp"]                      # uint8 [k,33]
         self.g_xy_canon = z["g_xy"]                  # uint8 [2048,64]
         self.h_xy_canon = z["h_xy"]

@@ -23,12 +23,14 @@ def _free_port():
 def _worker(rank, world, port, n, q):
     import sys
     sys.path.insert(0, ROOT)
+    sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
+    import srs_fixture
     os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port))
     dist.init_process_group("gloo", rank=rank, world_size=world)
     import proof_systems_b200 as zk
     from oracle import oracle as orc
     from proof_systems_b200.parallel import all_gather_point_sum, shard_bounds
-    z = np.load(os.path.join(ROOT, "tests", "golden", "vesta_srs.npz"))
+    z = srs_fixture.load("vesta", n)
     g = orc.decompress(orc.VESTA, z["g_cmp"][:n].tobytes())
     sc = orc.random_scalars(orc.FP, n, seed=3)
     lo, hi = shard_bounds(n, world, rank)

@@ -31,6 +31,20 @@ def test_writer_reproduces_the_reference_file(orc, pallas_srs, tmp_path):
     assert back.compressed and np.array_equal(back.g, pallas_srs.g_cmp) and np.array_equal(back.h, h) and not back.lagrange_bases
 
 
+@pytest.mark.parametrize("name", ["pallas", "vesta"])
+def test_rebuilt_generators_are_the_reference_ones(request, name):
+    """The fixture's 2^16 generators, rebuilt by tests/golden/srs_fixture.py, are byte for byte those of srs/<name>.srs, and the
+    stored selectors agree with the map's rule (the first candidate x whose x^3 + 5 is a square) on a sample."""
+    import srs_fixture
+    G = request.getfixturevalue(f"{name}_srs")
+    z = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", f"{name}_srs.npz"))
+    assert G.g_cmp.shape == (1 << 16, 33)
+    assert hashlib.sha256(G.g_cmp.tobytes()).digest() == z["g_cmp_sha256"].tobytes()
+    for i in list(range(64)) + [1000, 32768, 65535]:
+        xs = srs_fixture.candidate_xs(name, srs_fixture.map_input(i))
+        assert int(z["g_sel"][i]) & 3 == next(k for k, x in enumerate(xs) if srs_fixture.is_square(name, x))
+
+
 @pytest.mark.parametrize("name", ["pallas_srs", "vesta_srs"])
 def test_test_srs_layout_round_trip(request, name, tmp_path):
     """[g, h, {n: [[point]]}] with 65-byte uncompressed points, as srs/test_*.srs"""

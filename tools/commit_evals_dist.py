@@ -14,13 +14,15 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
+import srs_fixture
 import proof_systems_b200 as zk
 from oracle import oracle as orc
 
 LOG_N = 15
 n = 1 << LOG_N
 ctx = zk.Context(0)
-z = np.load(os.path.join(ROOT, "tests", "golden", "vesta_srs.npz"))
+z = srs_fixture.load("vesta")
 g = ctx.decompress_points(zk.VESTA, z["g_cmp"][:n]) if z["g_cmp"].shape[0] >= n else orc.extend_bases(orc.VESTA, ctx.decompress_points(zk.VESTA, z["g_cmp"]), n)
 h = orc.to_mont(orc.FQ, np.ascontiguousarray(z["h_xy"]).view("<u8").reshape(2, 4)).reshape(8)
 srs = zk.SRS(ctx, zk.VESTA, g, h)

@@ -4,9 +4,11 @@ import os, sys, threading, time
 import numpy as np
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
+import srs_fixture
 import proof_systems_b200 as zk
 from oracle import oracle as orc
-z = np.load(os.path.join(ROOT, "tests", "golden", "pallas_srs.npz"))
+z = srs_fixture.load("pallas")
 n, k = 1 << 14, 15
 c = zk.Context(0)
 g = c.decompress_points(zk.PALLAS, z["g_cmp"][:n])

@@ -5,6 +5,8 @@ import json, os, sys, threading, time
 import numpy as np, torch, torch.distributed as dist
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
+import srs_fixture
 import proof_systems_b200 as zk
 from proof_systems_b200.parallel import LibraryComm
 from bench import splitmix64_limbs
@@ -13,7 +15,7 @@ torch.cuda.set_device(local)
 dist.init_process_group("nccl", device_id=torch.device("cuda", local))
 ctx = zk.Context(local)
 stream = torch.cuda.Stream(); ctx.set_stream(stream.cuda_stream)
-z = np.load(os.path.join(ROOT, "tests", "golden", "pallas_srs.npz"))
+z = srs_fixture.load("pallas")
 g = ctx.decompress_points(zk.PALLAS, z["g_cmp"])
 n = 1 << 16
 bases = ctx.upload_bases(zk.PALLAS, g, window_bits=16)

@@ -9,12 +9,14 @@ import json, os, sys, time
 import numpy as np, torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
+import srs_fixture
 import proof_systems_b200 as zk
 from bench import splitmix64_limbs
 LOG_N = 16; N = 1 << LOG_N
 ctx = zk.Context(0)
 stream = torch.cuda.Stream(); ctx.set_stream(stream.cuda_stream)
-z = np.load(os.path.join(ROOT, "tests", "golden", "vesta_srs.npz"))
+z = srs_fixture.load("vesta")
 g = ctx.decompress_points(zk.VESTA, z["g_cmp"][:N])
 def timed(fn, reps=7):
     ts = []

@@ -10,10 +10,12 @@ sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import proof_systems_b200 as zk  # noqa: E402
 from bench import splitmix64_limbs  # noqa: E402
 
+sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "tests", "golden"))
+import srs_fixture  # noqa: E402
+
 
 def main():
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    z = np.load(os.path.join(root, "tests", "golden", "pallas_srs.npz"))
+    z = srs_fixture.load("pallas")
     ctx = zk.Context(0)
     g = ctx.decompress_points(zk.PALLAS, z["g_cmp"])
     n = g.shape[0]

@@ -5,12 +5,14 @@ import json, os, sys, time
 import numpy as np, torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
+import srs_fixture
 import proof_systems_b200 as zk
 from oracle import oracle as orc
 ctx = zk.Context(0)
 stream = torch.cuda.Stream(); ctx.set_stream(stream.cuda_stream)
 flush = torch.empty(256 << 20, dtype=torch.uint8, device="cuda")
-z = np.load(os.path.join(ROOT, "tests", "golden", "vesta_srs.npz"))
+z = srs_fixture.load("vesta")
 n = 1 << 20
 g = orc.extend_bases(orc.VESTA, ctx.decompress_points(zk.VESTA, z["g_cmp"]), n)
 sc = orc.random_scalars(orc.FP, n, seed=3)

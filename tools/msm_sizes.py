@@ -5,6 +5,8 @@ import json, os, sys
 import numpy as np, torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
+import srs_fixture
 import proof_systems_b200 as zk
 from bench import splitmix64_limbs
 ctx = zk.Context(0)
@@ -14,7 +16,7 @@ WINDOW = int(os.environ.get("MSM_WINDOW", "-1"))
 KS = [int(x) for x in os.environ.get("MSM_LOGS", "8,10,11,12,13,14,15,16").split(",")]
 stream = torch.cuda.Stream(); ctx.set_stream(stream.cuda_stream)
 flush = torch.empty(256 << 20, dtype=torch.uint8, device="cuda")
-z = np.load(os.path.join(ROOT, "tests", "golden", "pallas_srs.npz"))
+z = srs_fixture.load("pallas")
 g = ctx.decompress_points(zk.PALLAS, z["g_cmp"])
 def timed(fn, reps=7):
     ts = []

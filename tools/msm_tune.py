@@ -5,12 +5,14 @@ import json, os, sys
 import numpy as np, torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
+import srs_fixture
 import proof_systems_b200 as zk
 from bench import splitmix64_limbs
 ctx = zk.Context(0)
 stream = torch.cuda.Stream(); ctx.set_stream(stream.cuda_stream)
 flush = torch.empty(256 << 20, dtype=torch.uint8, device="cuda")
-z = np.load(os.path.join(ROOT, "tests", "golden", "pallas_srs.npz"))
+z = srs_fixture.load("pallas")
 g = ctx.decompress_points(zk.PALLAS, z["g_cmp"])
 LOG_N = int(os.environ.get("LOG_N", "16")); n = 1 << LOG_N
 def timed(fn, reps=9):

@@ -5,10 +5,12 @@ import numpy as np
 import torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
+import srs_fixture
 import proof_systems_b200 as zk
 from oracle import oracle as orc
 wb, chunk = int(sys.argv[1]), int(sys.argv[2])
-z = np.load(os.path.join(ROOT, "tests", "golden", "pallas_srs.npz"))
+z = srs_fixture.load("pallas")
 g = orc.decompress(orc.PALLAS, z["g_cmp"].tobytes())
 sc = orc.random_scalars(orc.FQ, 1 << 16, seed=1)
 ctx = zk.Context(0)

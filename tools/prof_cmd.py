@@ -5,6 +5,8 @@ import os, sys
 import numpy as np, torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
+import srs_fixture
 import proof_systems_b200 as zk
 from bench import splitmix64_limbs
 tma_ab = len(sys.argv) > 1 and sys.argv[1] == "msm_tma"      # alternate the two accumulate kernels (profiles/r02_tma_ab.md)
@@ -12,7 +14,7 @@ if tma_ab: sys.argv[1] = "16"
 wb = int(sys.argv[1]) if len(sys.argv) > 1 else 16
 reps = int(sys.argv[2]) if len(sys.argv) > 2 else 3
 ctx = zk.Context(0)
-z = np.load(os.path.join(ROOT, "tests", "golden", "pallas_srs.npz"))
+z = srs_fixture.load("pallas")
 g = ctx.decompress_points(zk.PALLAS, z["g_cmp"])
 bases = ctx.upload_bases(zk.PALLAS, g, window_bits=wb)
 d = torch.from_numpy(splitmix64_limbs(1, 1 << 16).view(np.int64)).cuda()

@@ -32,6 +32,8 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
+import srs_fixture
 
 LOG_N = int(os.environ.get("LOG_N", "16"))
 
@@ -48,7 +50,7 @@ def replay(zk, orc, ctx, log_n=LOG_N, check=True, n_open_polys=45):
     is compared with the oracle and an AssertionError names the first stage that differs."""
     N = 1 << log_n
     CID, FS = orc.VESTA, orc.FP
-    z = np.load(os.path.join(ROOT, "tests", "golden", "vesta_srs.npz"))
+    z = srs_fixture.load("vesta", N)
     assert z["g_cmp"].shape[0] >= N, "the fixture must hold all generators of the domain"
     g = ctx.decompress_points(zk.VESTA, z["g_cmp"][:N])
     h = orc.to_mont(orc.FQ, np.ascontiguousarray(z["h_xy"]).view("<u8").reshape(2, 4)).reshape(8)

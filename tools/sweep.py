@@ -12,6 +12,8 @@ import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
+sys.path.insert(0, os.path.join(ROOT, "tests", "golden"))
+import srs_fixture
 import proof_systems_b200 as zk
 from oracle import oracle as orc
 
@@ -38,7 +40,7 @@ def timed(fn, reps=5):
 
 which = sys.argv[1] if len(sys.argv) > 1 else "all"
 if which in ("all", "msm"):
-    z = np.load(os.path.join(ROOT, "tests", "golden", "pallas_srs.npz"))
+    z = srs_fixture.load("pallas")
     g = orc.decompress(orc.PALLAS, z["g_cmp"].tobytes())
     chunks = [int(x) for x in os.environ.get("CHUNKS", "16").split(",")]
     for log_n, windows in ((11, (0, 8, 10)), (16, (0, 12, 13, 14, 15, 16))):
