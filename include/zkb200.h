@@ -67,7 +67,9 @@ int zk_ctx_set_profile(zk_ctx* ctx, int enabled);
  *                "msm_batch": 1..16 MSMs of one call fused into ONE pipeline with one bucket group per MSM (zk_msm_batch,
  *                zk_srs_commit_non_hiding with several chunks, zk_srs_commit_evaluations_batch, the L/R pair of
  *                zk_ipa_round_lr): every latency-bound stage is paid once per batch; default 16.
- *                "msm_wave_threads": accumulation threads per SM the task count is sized for (0 = built-in default). */
+ *                "msm_wave_threads": accumulation threads per SM the task count is sized for (0 = built-in default).
+ *                "msm_pdl": 1 (default) launches the MSM pipeline's kernels after the first with programmatic dependent launch
+ *                and no per-call memsets; 0 uses plain launches behind two memsets (same results, for A/B timing). */
 int zk_ctx_set_option(zk_ctx* ctx, const char* name, long value);
 int zk_ctx_last_stage_ms(const zk_ctx* ctx, float* out, size_t capacity);
 

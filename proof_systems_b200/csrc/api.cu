@@ -215,6 +215,7 @@ int ctx_acquire_lane(zk_ctx* ctx, LaneLock& out) {
             c->parent = ctx;
             if (cudaSetDevice(ctx->device) != cudaSuccess || ctx_init_lane(c, ctx->device) != ZK_OK) { delete c; break; }
             c->batch = ctx->batch; c->ws.chunk = ctx->ws.chunk; c->ws.wave_threads = ctx->ws.wave_threads; c->ws.tma_gather = ctx->ws.tma_gather;
+            c->ws.pdl = ctx->ws.pdl;
             ctx->children.push_back(c);
         }
         lanes.push_back(ctx);
@@ -393,6 +394,12 @@ int zk_ctx_set_option(zk_ctx* ctx, const char* name, long value) {
         if (value < 0 || value > 1) { zk_set_error("set_option: msm_tma %ld outside [0, 1]", value); return ZK_ERR_INVALID; }
         ctx->ws.tma_gather = value != 0;
         for (zk_ctx* c : ctx->children) c->ws.tma_gather = value != 0;
+        return ZK_OK;
+    }
+    if (!strcmp(name, "msm_pdl")) {
+        if (value < 0 || value > 1) { zk_set_error("set_option: msm_pdl %ld outside [0, 1]", value); return ZK_ERR_INVALID; }
+        ctx->ws.pdl = value != 0;
+        for (zk_ctx* c : ctx->children) c->ws.pdl = value != 0;
         return ZK_OK;
     }
     if (!strcmp(name, "msm_wave_threads")) {

@@ -86,6 +86,22 @@ void msm_bases_free(MsmBases& b) {
     b = MsmBases();
 }
 
+// ---------------------------------------------------------------------------------------------- launch chain
+// Every kernel of msm_run after the first is launched with programmatic dependent launch (PDL): its CTAs may become resident while
+// the previous kernel's last CTAs still run, and wait in pdl_wait() (griddepcontrol.wait) until that kernel has completed and its
+// stores are visible.  Two rules make every read of the pipeline ordered:
+//   (1) every thread of every kernel after the first executes pdl_wait() before it exits, triggers, or reads the previous kernel's
+//       output, and writes no global memory before it.  (The first, k_recode, is an ordinary launch: it starts after everything
+//       before it on the stream, the previous call's kernels included.)  So kernel N completes only after kernel N-1 has completed, and by
+//       induction after every earlier kernel: reads after the wait see the output of ANY earlier kernel (gridsum reading buckets
+//       written by accumulate or the finish kernels, bucket_finish reading offsets from plan, ...);
+//   (2) kernel N is launched only once every CTA of kernel N-1 has triggered or exited, which by (1) is after N-1's wait, i.e.
+//       after kernel N-2 completed.  So the prologue BEFORE the wait may read what kernel N-2 or earlier wrote: the plan's
+//       offsets, task_off and meta in accumulate, run_sum and bucket_finish (plan is at least two kernels back there).
+// Without the PDL attribute (profile mode, option msm_pdl = 0) both instructions are no-ops and stream order applies.
+__device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
+__device__ __forceinline__ void pdl_trigger() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
+
 // ---------------------------------------------------------------------------------------------- recode + histogram
 // One thread per scalar of one MSM of the batch (blockIdx.y): Montgomery -> canonical if asked (VariableBaseMSM::msm ==
 // into_bigint + msm_bigint), then signed base-2^c digits d_w in (-2^(c-1), 2^(c-1)]; digit w of scalar i of MSM j at
@@ -121,6 +137,7 @@ __global__ void k_recode(MsmScalarSet sc, int scalars_mont, size_t n, unsigned c
         const uint32_t peers = __match_any_sync(__activemask(), key);
         if (sd != 0 && (threadIdx.x & 31) == (unsigned)(__ffs(peers) - 1)) atomicAdd(&counts[key], (uint32_t)__popc(peers));
     }
+    pdl_trigger();
 }
 
 // Planning pass over the histogram: exclusive scans of the bucket counts (-> offsets of the sorted entry list) and of the
@@ -128,7 +145,9 @@ __global__ void k_recode(MsmScalarSet sc, int scalars_mont, size_t n, unsigned c
 // spins on tile t-1's published inclusive total — tiles are dispatched in order, so the predecessor is always resident), which
 // keeps the scan a single launch for any batch size.  64-bit lanes carry (entry count << 32 | task count): one scan yields both.
 // Buckets with more than smax tasks ("giant": the all-ones witness columns of kimchi put ~n entries in one bucket,
-// SURVEY.md §3.1) are listed for k_giant_finish.  Clears counts (re-used as scatter cursors).
+// SURVEY.md §3.1) are listed for k_giant_finish.  Empty buckets get the identity here (all-zero XYZZ): every other bucket is
+// written by exactly one of k_accumulate (one task), k_giant_finish, k_bucket_finish(_serial).  The counts stay: k_scatter
+// counts them down to zero as its cursors, so every call finds them zeroed.
 __device__ __forceinline__ uint64_t block_excl_scan_1024(uint64_t v, uint64_t* warp_sums, uint64_t* tile_total) {
     const unsigned tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
     uint64_t x = v;
@@ -157,17 +176,19 @@ __device__ __forceinline__ uint64_t block_excl_scan_1024(uint64_t v, uint64_t* w
 
 constexpr unsigned PLAN_PER_THREAD = 4, PLAN_TILE = 1024 * PLAN_PER_THREAD;
 __global__ void __launch_bounds__(1024) k_plan(uint32_t* counts, uint32_t* offsets, uint32_t* task_off, uint32_t nb, uint32_t K, uint32_t smax,
-                                                 uint32_t* meta, uint32_t* giants, uint64_t* chain, uint32_t* chain_flag, uint32_t epoch) {
+                                                 uint32_t* meta, uint32_t* giants, uint64_t* chain, uint32_t* chain_flag, uint32_t epoch,
+                                                 xyzz_t* buckets) {
     __shared__ uint64_t warp_sums[32];
     __shared__ uint64_t tile_total, prefix_s;
     const unsigned tid = threadIdx.x, tile = blockIdx.x;
     const uint32_t i0 = tile * PLAN_TILE + tid * PLAN_PER_THREAD;
     uint32_t v[PLAN_PER_THREAD];
     uint64_t pk[PLAN_PER_THREAD], sum = 0;
+    pdl_wait();
 #pragma unroll
     for (unsigned k = 0; k < PLAN_PER_THREAD; k++) {
         v[k] = i0 + k < nb ? counts[i0 + k] : 0;
-        if (i0 + k < nb) counts[i0 + k] = 0;
+        if (i0 + k < nb && v[k] == 0) store_xyzz(buckets + i0 + k, xyzz_identity());
         pk[k] = ((uint64_t)v[k] << 32) | ((v[k] + K - 1) / K);
         sum += pk[k];
     }
@@ -204,14 +225,17 @@ __global__ void __launch_bounds__(1024) k_plan(uint32_t* counts, uint32_t* offse
         offsets[nb] = (uint32_t)(tot >> 32); task_off[nb] = (uint32_t)tot;
         meta[0] = (uint32_t)(tot >> 32); meta[1] = (uint32_t)tot;
     }
+    pdl_trigger();
 }
 
-// Counting-sort scatter: entry (point index | sign) of every non-zero digit goes to its bucket's range.
+// Counting-sort scatter: entry (point index | sign) of every non-zero digit goes to its bucket's range.  The cursors are the
+// histogram, counted DOWN: a bucket's slots are handed out from its end, and the counts are zero again when the kernel ends.
 __global__ void k_scatter(const int32_t* digits, size_t n, unsigned c, unsigned nwin, unsigned batch, unsigned gpm, int per_window, MsmScalarSet sc,
                           size_t table_stride, int use_table, size_t n_main, size_t n_extra, uint32_t main_count, const uint32_t* offsets,
                           uint32_t* cursors, uint32_t* entries) {
     size_t id = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     const bool in_range = id < n * nwin * batch;
+    pdl_wait();
     int32_t sd = in_range ? digits[id] : 0;
     const unsigned jw = (unsigned)(id / n), j = jw / nwin, w = jw - j * nwin;
     size_t i = id - (size_t)jw * n;
@@ -222,7 +246,7 @@ __global__ void k_scatter(const int32_t* digits, size_t n, unsigned c, unsigned 
     const uint32_t peers = __match_any_sync(0xffffffffu, key);
     const unsigned lane = threadIdx.x & 31, leader = (unsigned)(__ffs(peers) - 1);
     uint32_t base = 0;
-    if (sd != 0 && lane == leader) base = atomicAdd(&cursors[key], (uint32_t)__popc(peers));
+    if (sd != 0 && lane == leader) base = atomicSub(&cursors[key], (uint32_t)__popc(peers)) - (uint32_t)__popc(peers);
     base = __shfl_sync(0xffffffffu, base, leader);
     if (sd == 0) return;
     uint32_t pos = offsets[key] + base + (uint32_t)__popc(peers & ((1u << lane) - 1));
@@ -230,6 +254,7 @@ __global__ void k_scatter(const int32_t* digits, size_t n, unsigned c, unsigned 
     size_t pidx = i < n_main ? (use_table ? (size_t)w * table_stride : 0) + sc.off[in_range ? j : 0] + i
                              : (size_t)main_count + (use_table ? (size_t)w * n_extra : 0) + (i - n_main);
     entries[pos] = (uint32_t)pidx | (sd < 0 ? 0x80000000u : 0u);
+    pdl_trigger();
 }
 
 // ---------------------------------------------------------------------------------------------- accumulation
@@ -242,13 +267,16 @@ __global__ void __launch_bounds__(128) k_accumulate(const affine_t* __restrict__
                                                     uint32_t K, const uint32_t* __restrict__ meta, const affine_t* __restrict__ extra,
                                                     uint32_t main_count, xyzz_t* buckets, xyzz_t* partials) {
     const uint32_t t = blockIdx.x * blockDim.x + threadIdx.x;
-    if (t >= __ldg(meta + 1)) return;
+    // prologue: the plan (two kernels back) is complete when this grid launches
+    const bool live = t < __ldg(meta + 1);
     // upper_bound(task_off[0..nb], t) - 1
     uint32_t lo = 0, hi = nb;  // invariant: task_off[lo] <= t < task_off[hi]
-    while (hi - lo > 1) {
+    while (live && hi - lo > 1) {
         uint32_t mid = (lo + hi) >> 1;
         if (__ldg(task_off + mid) <= t) lo = mid; else hi = mid;
     }
+    pdl_wait();                // the entries of k_scatter
+    if (!live) return;
     const uint32_t b = lo;
     const uint32_t e0 = __ldg(offsets + b), nbk = __ldg(offsets + b + 1) - e0;
     const uint32_t sb = (nbk + K - 1) / K, sub = t - __ldg(task_off + b);
@@ -273,6 +301,7 @@ __global__ void __launch_bounds__(128) k_accumulate(const affine_t* __restrict__
         acc = xyzz_madd<F>(acc, q);
     }
     store_xyzz(sb == 1 ? buckets + b : partials + t, acc);
+    pdl_trigger();
 }
 
 // ---------------------------------------------------------------------------------------------- accumulation, TMA-staged gather
@@ -324,6 +353,7 @@ __global__ void __launch_bounds__(128) k_accumulate_tma(const affine_t* __restri
         i = e0 + sub * base + min(sub, rem);
         end = i + base + (sub < rem ? 1u : 0u);
     }
+    pdl_wait();                // the entries of k_scatter (the prologue above reads the plan only, see k_accumulate)
     const uint32_t steps = __reduce_max_sync(0xffffffffu, end - i);
     uint32_t sign[2] = {0, 0};
     auto issue = [&](uint32_t step) {
@@ -356,6 +386,7 @@ __global__ void __launch_bounds__(128) k_accumulate_tma(const affine_t* __restri
         }
     }
     if (live) store_xyzz(sb == 1 ? buckets + b : partials + t, acc);
+    pdl_trigger();
 }
 
 // Balanced first level of the per-bucket sums.  The task partials lie in bucket order; thread u sums the RUN of `run`
@@ -367,10 +398,10 @@ __global__ void __launch_bounds__(128) k_accumulate_tma(const affine_t* __restri
 template <class F>
 __global__ void __launch_bounds__(128, 4) k_run_sum(const uint32_t* __restrict__ task_off, uint32_t nb, const uint32_t* __restrict__ meta, uint32_t run,
                                                  uint32_t smax, xyzz_t* partials) {
+    // prologue: the plan's task_off and meta (three kernels back) are complete when this grid launches
     const uint32_t nt = meta[1];
     const uint64_t i0w = (uint64_t)(blockIdx.x * blockDim.x + threadIdx.x) * run;
-    if (i0w >= nt) return;
-    const uint32_t i0 = (uint32_t)i0w, i1 = min(nt, i0 + run);
+    const uint32_t i0 = i0w < nt ? (uint32_t)i0w : nt, i1 = min(nt, i0 + run);
     // largest b with task_off[b] <= i0 (skips the empty buckets that share a start)
     uint32_t lo = 0, hi = nb;
     while (hi - lo > 1) {
@@ -381,7 +412,8 @@ __global__ void __launch_bounds__(128, 4) k_run_sum(const uint32_t* __restrict__
     // giant buckets were summed by k_giant_finish: their slots are skipped (a thread wholly inside one does nothing)
     const bool giants_done = meta[2] <= MSM_MAX_GIANTS;
     bool skip = giants_done && nxt - __ldg(task_off + b) > smax;
-    if (skip && nxt >= i1) return;
+    pdl_wait();                // the partials of k_accumulate, read after k_giant_finish has read them
+    if (i0w >= nt || (skip && nxt >= i1)) return;
     xyzz_t acc = load_xyzz(partials + i0);
     bool dirty = false;
     for (uint32_t i = i0 + 1; i < i1; i++) {
@@ -407,6 +439,7 @@ __global__ void __launch_bounds__(128, 4) k_run_sum(const uint32_t* __restrict__
         }
     }
     if (dirty) store_xyzz(partials + seg, acc);
+    pdl_trigger();
 }
 
 // Thread-per-bucket finish pass, for MANY buckets with few partials each: with more buckets than resident quads the pass is
@@ -417,12 +450,16 @@ __global__ void __launch_bounds__(128, 4) k_bucket_finish_serial(const uint32_t*
                                                               uint32_t K, uint32_t smax, const uint32_t* __restrict__ meta, uint32_t run, xyzz_t* buckets,
                                                               const xyzz_t* __restrict__ partials) {
     const uint32_t b = blockIdx.x * blockDim.x + threadIdx.x;
-    if (b >= nb) return;
-    const uint32_t nbk = __ldg(offsets + b + 1) - __ldg(offsets + b);
-    uint32_t sb = (nbk + K - 1) / K;
-    if (sb > smax && meta[2] <= MSM_MAX_GIANTS) return;  // k_giant_finish
-    if (sb < 2) return;                                  // 0: empty, 1: written by k_accumulate
-    const uint32_t a = __ldg(task_off + b);
+    // prologue: the plan's offsets, task_off and meta (at least three kernels back) are complete when this grid launches
+    uint32_t sb = 0, a = 0;
+    if (b < nb) {
+        const uint32_t nbk = __ldg(offsets + b + 1) - __ldg(offsets + b);
+        sb = (nbk + K - 1) / K;
+        if (sb > smax && meta[2] <= MSM_MAX_GIANTS) sb = 0;  // k_giant_finish
+        a = __ldg(task_off + b);
+    }
+    pdl_wait();                                              // the partials of k_run_sum (or k_accumulate)
+    if (sb < 2) return;                                      // 0: empty, 1: written by k_accumulate
     xyzz_t acc = load_xyzz(partials + a);
     if (run == 0) {
         for (uint32_t j = 1; j < sb; j++) acc = xyzz_add<F, true>(acc, load_xyzz(partials + a + j));
@@ -430,6 +467,7 @@ __global__ void __launch_bounds__(128, 4) k_bucket_finish_serial(const uint32_t*
         for (uint32_t k = (a / run + 1) * run; k < a + sb; k += run) acc = xyzz_add<F, true>(acc, load_xyzz(partials + k));
     }
     store_xyzz(buckets + b, acc);
+    pdl_trigger();
 }
 
 // Buckets with 2 <= s_b <= smax tasks: a group of G = 2^log_g QUADS (quad.cuh) sums the bucket's partials — strided serial
@@ -449,6 +487,7 @@ __global__ void __launch_bounds__(128) k_bucket_finish(const uint32_t* __restric
         if (sb > smax && meta[2] <= MSM_MAX_GIANTS) sb = 0;
         if (sb < 2) sb = 0;
     }
+    pdl_wait();                // the prologue above reads the plan only (at least two kernels back); the partials come from k_accumulate
     // warp-uniform trip count: every lane must take part in the quad additions' shuffles
     const unsigned my_trips = sb > gl ? (sb - gl + G - 1) / G : 0;
     const unsigned trips = __reduce_max_sync(0xffffffffu, my_trips);
@@ -465,6 +504,7 @@ __global__ void __launch_bounds__(128) k_bucket_finish(const uint32_t* __restric
         acc = xyzz_add_quad<F>(acc, o);
     }
     if (gl == 0 && sb && (threadIdx.x & 3) == 0) store_xyzz(buckets + b, acc);
+    pdl_trigger();
 }
 
 // ---------------------------------------------------------------------------------------------- bucket reduction
@@ -483,6 +523,7 @@ __global__ void __launch_bounds__(TREE_THREADS) k_giant_finish(const uint32_t* _
                                                                uint32_t* tickets) {
     extern __shared__ xyzz_t sm_tree[];
     __shared__ uint32_t ticket_s;
+    pdl_wait();                // the partials of k_accumulate
     const uint32_t ng = meta[2];
     if (ng > MSM_MAX_GIANTS || blockIdx.x >= ng) return;  // overflow: k_bucket_finish took them
     const uint32_t b = giants[blockIdx.x];
@@ -508,6 +549,7 @@ __global__ void __launch_bounds__(TREE_THREADS) k_giant_finish(const uint32_t* _
     acc = qd < GIANT_SLICES ? load_xyzz(mine + qd) : xyzz_identity();
     acc = block_tree_sum_quad<F>(acc, sm_tree);
     if (threadIdx.x == 0) { store_xyzz(buckets + b, acc); tickets[blockIdx.x] = 0; }
+    pdl_trigger();
 }
 
 // Two-level form of the same reduction (fewer additions, shorter dependency chains).  Split i = hi * W + lo, W = 2^w_lo:
@@ -540,6 +582,7 @@ __global__ void __launch_bounds__(128, 3) k_gridsum(const xyzz_t* __restrict__ b
         }
         return part;
     };
+    pdl_wait();                // the buckets: k_plan, k_accumulate, k_giant_finish and the finish kernels all wrote some
     fe nxt = fetch(qd);
     for (uint32_t e0 = 0; e0 < count; e0 += nq) {
         xyzz_t o;
@@ -549,6 +592,7 @@ __global__ void __launch_bounds__(128, 3) k_gridsum(const xyzz_t* __restrict__ b
     }
     acc = block_tree_sum_quad<F>(acc, sm_tree);
     if (threadIdx.x == 0) store_xyzz(rc + (size_t)g * (nrows + W) + blockIdx.x, acc);
+    pdl_trigger();
 }
 
 template <class F>
@@ -562,6 +606,7 @@ __global__ void __launch_bounds__(TREE_THREADS) k_gridsum_final(const xyzz_t* __
     const unsigned bit = cols ? t : t - w_lo;
     const unsigned qd = threadIdx.x >> 2, nq = blockDim.x >> 2;
     xyzz_t acc = xyzz_identity();
+    pdl_wait();                // the row / column sums of k_gridsum
     // the j-th index with `bit` set: e = (j >> bit) << (bit + 1) | 1 << bit | (j & (2^bit - 1))
     for (uint32_t j0 = 0;; j0 += nq) {
         const uint32_t first = ((j0 >> bit) << (bit + 1)) | (1u << bit) | (j0 & ((1u << bit) - 1));
@@ -584,6 +629,18 @@ void msm_workspace_free(MsmWorkspace& ws) {
     if (ws.h_bitsums) cudaFreeHost(ws.h_bitsums);
     for (auto& e : ws.ev) if (e) cudaEventDestroy(e);
     ws = MsmWorkspace();
+}
+
+// a kernel launch on `st`; pdl: programmatic stream serialization with the kernel before it (see "launch chain" above)
+template <class... KArgs, class... Args>
+static cudaError_t launch(bool pdl, void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st, Args&&... args) {
+    cudaLaunchAttribute attr;
+    attr.id = cudaLaunchAttributeProgrammaticStreamSerialization;
+    attr.val.programmaticStreamSerializationAllowed = 1;
+    cudaLaunchConfig_t cfg = {};
+    cfg.gridDim = grid; cfg.blockDim = block; cfg.dynamicSmemBytes = smem; cfg.stream = st;
+    cfg.attrs = &attr; cfg.numAttrs = pdl ? 1 : 0;
+    return cudaLaunchKernelEx(&cfg, kern, std::forward<Args>(args)...);
 }
 
 static unsigned pow2_ceil_log(uint64_t x) {
@@ -670,6 +727,7 @@ int msm_run(const MsmBases& b, const size_t* offs, size_t n_main, const fe* cons
             free_dev(ws.d_counts); free_dev(ws.d_offsets); free_dev(ws.d_task_off); free_dev(ws.d_buckets); free_dev(ws.d_chain); free_dev(ws.d_chain_flag);
             ws.d_counts = ws.d_offsets = ws.d_task_off = ws.d_chain_flag = nullptr; ws.d_chain = nullptr; ws.d_buckets = nullptr; ws.cap_buckets = 0;
             ZK_CUDA(cudaMalloc(&ws.d_counts, NB * sizeof(uint32_t)));
+            ZK_CUDA(cudaMemsetAsync(ws.d_counts, 0, NB * sizeof(uint32_t), st));   // then kept zero by k_scatter
             ZK_CUDA(cudaMalloc(&ws.d_offsets, (NB + 1) * sizeof(uint32_t)));
             ZK_CUDA(cudaMalloc(&ws.d_task_off, (NB + 1) * sizeof(uint32_t)));
             ZK_CUDA(cudaMalloc(&ws.d_buckets, NB * sizeof(xyzz_t)));
@@ -709,41 +767,44 @@ int msm_run(const MsmBases& b, const size_t* offs, size_t n_main, const fe* cons
     MsmScalarSet sc{};
     for (unsigned j = 0; j < k; j++) { sc.p[j] = d_scalars[j]; sc.off[j] = (uint32_t)offs[j]; }
     const uint32_t epoch = ++ws.epoch;
-    ZK_CUDA(cudaMemsetAsync(ws.d_counts, 0, NB * sizeof(uint32_t), st));
-    ZK_CUDA(cudaMemsetAsync(ws.d_buckets, 0, NB * sizeof(xyzz_t), st));  // all-zero XYZZ == identity
+    if (!ws.pdl) {
+        // the launch shell this pipeline had before the PDL chain, kept for A/B (option msm_pdl = 0): both memsets are redundant
+        ZK_CUDA(cudaMemsetAsync(ws.d_counts, 0, NB * sizeof(uint32_t), st));
+        ZK_CUDA(cudaMemsetAsync(ws.d_buckets, 0, NB * sizeof(xyzz_t), st));
+    }
+    // kernels 2.. wait for their predecessor in-kernel; profile mode launches plainly so that the stage events bracket one kernel each
+    const bool pdl = ws.pdl && !ws.profile;
     STAGE_MARK(0);
-    // 1. digits + histogram
+    // 1. digits + histogram (an ordinary launch: it follows everything before it on the stream, the previous call included)
     k_recode<FS><<<dim3((unsigned)((n + 127) / 128), k), 128, 0, st>>>(sc, scalars_mont ? 1 : 0, n, c, nwin, gpm, use_table ? 0 : 1, ws.d_digits,
                                                                         ws.d_counts, ws.d_meta);
     STAGE_MARK(1);
-    // 2. plan: bucket offsets, task offsets, giant list
-    k_plan<<<(unsigned)ntiles, 1024, 0, st>>>(ws.d_counts, ws.d_offsets, ws.d_task_off, (uint32_t)NB, K, smax, ws.d_meta, ws.d_giants, ws.d_chain,
-                                               ws.d_chain_flag, epoch);
+    // 2. plan: bucket offsets, task offsets, giant list, identity of the empty buckets
+    ZK_CUDA(launch(pdl, k_plan, dim3((unsigned)ntiles), dim3(1024), 0, st, ws.d_counts, ws.d_offsets, ws.d_task_off, (uint32_t)NB, K, smax, ws.d_meta,
+                   ws.d_giants, ws.d_chain, ws.d_chain_flag, epoch, ws.d_buckets));
     STAGE_MARK(2);
     // 3. scatter (counting sort by bucket)
-    k_scatter<<<(unsigned)((Mmax + 255) / 256), 256, 0, st>>>(ws.d_digits, n, c, nwin, k, gpm, use_table ? 0 : 1, sc, b.n, use_table ? 1 : 0,
-                                                            n_main, n_extra, (uint32_t)main_count, ws.d_offsets, ws.d_counts, ws.d_entries);
+    ZK_CUDA(launch(pdl, k_scatter, dim3((unsigned)((Mmax + 255) / 256)), dim3(256), 0, st, ws.d_digits, n, c, nwin, k, gpm, use_table ? 0 : 1, sc, b.n,
+                   use_table ? 1 : 0, n_main, n_extra, (uint32_t)main_count, ws.d_offsets, ws.d_counts, ws.d_entries));
     STAGE_MARK(3);
     // 4. accumulation: one task per <= K sorted entries of one bucket
-    if (ws.tma_gather)
-        k_accumulate_tma<F><<<(unsigned)((NTmax + 127) / 128), 128, 0, st>>>(b.d_points, ws.d_entries, ws.d_offsets, ws.d_task_off, (uint32_t)NB, K,
-                                                                           ws.d_meta, d_extra, (uint32_t)main_count, ws.d_buckets, ws.d_partials);
-    else
-        k_accumulate<F><<<(unsigned)((NTmax + 127) / 128), 128, 0, st>>>(b.d_points, ws.d_entries, ws.d_offsets, ws.d_task_off, (uint32_t)NB, K, ws.d_meta,
-                                                                       d_extra, (uint32_t)main_count, ws.d_buckets, ws.d_partials);
+    ZK_CUDA(launch(pdl, ws.tma_gather ? k_accumulate_tma<F> : k_accumulate<F>, dim3((unsigned)((NTmax + 127) / 128)), dim3(128), 0, st, b.d_points,
+                   ws.d_entries, ws.d_offsets, ws.d_task_off, (uint32_t)NB, K, ws.d_meta, d_extra, (uint32_t)main_count, ws.d_buckets, ws.d_partials));
     STAGE_MARK(4);
     // 5. per-bucket sums of the task partials (+ giants)
     // giants first: k_giant_finish reads the untouched partial lists, k_run_sum then rewrites partials in place
-    k_giant_finish<F><<<dim3(64, GIANT_SLICES), TREE_THREADS, TREE_QUADS * sizeof(xyzz_t), st>>>(
-        ws.d_giants, ws.d_meta, ws.d_offsets, ws.d_task_off, K, ws.d_buckets, ws.d_partials, ws.d_giant_slices, ws.d_giant_tickets);
+    ZK_CUDA(launch(pdl, k_giant_finish<F>, dim3(64, GIANT_SLICES), dim3(TREE_THREADS), TREE_QUADS * sizeof(xyzz_t), st, ws.d_giants, ws.d_meta,
+                   ws.d_offsets, ws.d_task_off, K, ws.d_buckets, ws.d_partials, ws.d_giant_slices, ws.d_giant_tickets));
     if (serial_finish) {
         const size_t threads = (NTmax + run - 1) / run;
-        k_run_sum<F><<<(unsigned)((threads + 127) / 128), 128, 0, st>>>(ws.d_task_off, (uint32_t)NB, ws.d_meta, run, smax, ws.d_partials);
+        ZK_CUDA(launch(pdl, k_run_sum<F>, dim3((unsigned)((threads + 127) / 128)), dim3(128), 0, st, ws.d_task_off, (uint32_t)NB, ws.d_meta, run, smax,
+                       ws.d_partials));
         nl += 1;
-        k_bucket_finish_serial<F><<<(unsigned)((NB + 127) / 128), 128, 0, st>>>(ws.d_offsets, ws.d_task_off, (uint32_t)NB, K, smax, ws.d_meta, run, ws.d_buckets, ws.d_partials);
+        ZK_CUDA(launch(pdl, k_bucket_finish_serial<F>, dim3((unsigned)((NB + 127) / 128)), dim3(128), 0, st, ws.d_offsets, ws.d_task_off, (uint32_t)NB, K,
+                       smax, ws.d_meta, run, ws.d_buckets, ws.d_partials));
     } else {
-        k_bucket_finish<F><<<(unsigned)(((NB << (log_g + 2)) + 127) / 128), 128, 0, st>>>(ws.d_offsets, ws.d_task_off, (uint32_t)NB, K, smax, log_g, ws.d_meta,
-                                                                                  ws.d_buckets, ws.d_partials);
+        ZK_CUDA(launch(pdl, k_bucket_finish<F>, dim3((unsigned)(((NB << (log_g + 2)) + 127) / 128)), dim3(128), 0, st, ws.d_offsets, ws.d_task_off,
+                       (uint32_t)NB, K, smax, log_g, ws.d_meta, ws.d_buckets, ws.d_partials));
     }
     STAGE_MARK(5);
     // 6. two-level bucket reduction: row / column sums of the bucket grid, then their bit slices
@@ -754,10 +815,10 @@ int msm_run(const MsmBases& b, const size_t* offs, size_t n_main, const fe* cons
         // SM at the kernel's register budget), so that the whole grid of a single MSM — 385 CTAs at window 16 — runs as one wave
         unsigned gt = 128;                          // k_gridsum is built for 3 CTAs of 128 threads per SM (<= 168 registers)
         while (gt > 32 && (gt / 4 >= 2 * std::max(W, nrows) || (size_t)G * (nrows + W) * gt > (size_t)ws.sm_count * 384)) gt /= 2;
-        k_gridsum<F><<<dim3(nrows + W, 1, G), gt, (gt / 4) * sizeof(xyzz_t), st>>>(ws.d_buckets, B, w_lo, d_rc);
+        ZK_CUDA(launch(pdl, k_gridsum<F>, dim3(nrows + W, 1, G), dim3(gt), (gt / 4) * sizeof(xyzz_t), st, ws.d_buckets, B, w_lo, d_rc));
         unsigned ft = TREE_THREADS;                 // half of the elements carry a given bit
         while (ft > 32 && ft / 4 >= std::max(W, nrows)) ft /= 2;
-        k_gridsum_final<F><<<dim3(c, G), ft, (ft / 4) * sizeof(xyzz_t), st>>>(d_rc, B, w_lo, c, d_T);
+        ZK_CUDA(launch(pdl, k_gridsum_final<F>, dim3(c, G), dim3(ft), (ft / 4) * sizeof(xyzz_t), st, d_rc, B, w_lo, c, d_T));
     }
     nl += 8;
     STAGE_MARK(6);

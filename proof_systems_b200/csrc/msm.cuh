@@ -54,7 +54,7 @@ struct MsmWorkspace {
     int32_t* d_digits = nullptr;      // [k][nwin][n]
     uint32_t* d_entries = nullptr;    // [M]  point index | sign << 31, sorted by bucket
     xyzz_t* d_partials = nullptr;     // [tasks] one partial sum per accumulation task
-    uint32_t* d_counts = nullptr;     // [NB]     histogram, then scatter cursors
+    uint32_t* d_counts = nullptr;     // [NB]     histogram, then scatter cursors counting down: zero between calls
     uint32_t* d_offsets = nullptr;    // [NB + 1] exclusive scan of the counts
     uint32_t* d_task_off = nullptr;   // [NB + 1] exclusive scan of ceil(count / K)
     xyzz_t* d_buckets = nullptr;      // [NB]
@@ -74,6 +74,8 @@ struct MsmWorkspace {
     uint32_t chunk = 0;               // K override (0: chosen per call so that the tasks fill the machine once)
     uint32_t wave_threads = 0;        // accumulation threads per SM the task count is sized for (0: built-in default)
     bool tma_gather = false;          // A/B switch: gather the points with the bulk asynchronous copy engine (k_accumulate_tma)
+    bool pdl = true;                  // A/B switch: kernels 2.. by programmatic dependent launch, no per-call memsets (false: plain
+                                      // launches behind two memsets, the earlier launch shell)
     int sm_count = 148;               // SMs of the device (set by the context)
     bool profile = false;             // record an event after every stage
     cudaEvent_t ev[8] = {};           // MSM_ST_COUNT + 1 stage boundaries
